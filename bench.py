@@ -2,6 +2,7 @@
 """bench.py -- dual-simplex iterations/sec (and wall-to-optimal) of the B200 engine on BASELINE.json's workloads.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|small]
+                  [--dump-outputs DIR]
 
 Workloads
   N = 1 (default c2): BASELINE.json configs[1] -- synthetic random LP m=10k n=100k 1% nnz, fp64, dual
@@ -21,6 +22,11 @@ Workloads
 
 W warm-up steps run untimed, then exactly K steps are timed with CUDA events on the engine's stream
 (max over ranks).
+
+--dump-outputs DIR writes what the timed call hands its caller after the last timed step -- primal and
+dual column / row solutions, the status array and the objective -- as DIR/<name>.npy (rank 0).  The
+inputs are generated from fixed seeds and start from a committed basis, so two builds run with the
+same arguments can be compared output for output.
 
 --impl reference times the reference's CPU implementation of the path.  coin-or/Clp cannot be built
 here (its CoinUtils dependency is absent), so the arm runs the CPU restatement in oracle/
@@ -314,6 +320,18 @@ def run_reference(args, name, lp, status, start, cycle):
     }
 
 
+def dump_outputs(path, s):
+    """The arrays a caller of the timed dual() receives, in float64 (status codes in float32): 2.2 MB at
+    c2 and 11 MB at c3, so every entry is written."""
+    os.makedirs(path, exist_ok=True)
+    outputs = {"primalColumnSolution": s.primalColumnSolution(), "primalRowSolution": s.primalRowSolution(),
+               "dualColumnSolution": s.dualColumnSolution(), "dualRowSolution": s.dualRowSolution(),
+               "statusArray": s.statusArray().astype(np.float32),
+               "objectiveValue": np.array([s.objectiveValue()], dtype=np.float64)}
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def _claim_stdout():
     """Rank 0 must print exactly ONE JSON line: park the real stdout and point fd 1 at stderr, so that
     library banners (NCCL prints its version to stdout) cannot precede or follow the line."""
@@ -335,7 +353,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
     ap.add_argument("--no-optimal", action="store_true", help="skip the solve-to-optimality leg (N=1, c2)")
     ap.add_argument("--save-status", default=None, help="write the status array after the run (fixture generation)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the timed call after its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path; the reference arm only samples the window")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else max(args.warmup, 1)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -420,6 +442,8 @@ def main():
     nucleus = s.nucleusSize()
     if args.save_status and rank == 0:
         np.savez_compressed(args.save_status, status=s.statusArray(), iterations=s.numberIterations())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, s)
 
     result = {
         "metric": "dual_simplex_iterations_per_sec", "value": value, "unit": "iterations/s",

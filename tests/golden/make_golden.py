@@ -1,10 +1,11 @@
-"""Freeze the reference's known-answer LPs into fixtures (run in the build container).
+"""Freeze the reference's known-answer LPs into fixtures.
 
-Sources (all under /root/reference, read-only):
-  * test/test_racing_lp.cpp generators (glibc srand/rand) + test/test_racing_reference.txt
-    expected LP bounds -> <name>.npz with known_objective
+Sources (files of coin-or/Clp):
+  * test/test_racing_lp.cpp generators (glibc srand/rand, restated in clp_b200/generators.py) +
+    test/test_racing_reference.txt expected LP bounds -> <name>.npz with known_objective
   * src/unitTest.cpp:1415-1431 3x5 LP -> unitTest-3x5.npz
-  * examples/modified_afiro.mps, examples/hello.mps parsed with THIS repo's MPS reader ->
+  * examples/modified_afiro.mps, examples/hello.mps (copied verbatim next to this script) parsed
+    with THIS repo's MPS reader ->
     .npz (no reference value is printed for them; the expected objective stored is the
     independent HiGHS dual simplex optimum, see SURVEY.md 8c item 3)
 Every fixture without a reference-published objective gets `known_objective` from HiGHS
@@ -52,17 +53,16 @@ def main():
     # no reference value exists for them: pinned by HiGHS dual simplex, cross-checked by the oracle
     cases += [G.staircase_lp(8, 60, 3), G.staircase_lp(10, 100, 4), G.transportation_lp(10, 200, 5),
               G.transportation_lp(20, 500, 6)]
-    # in-tree MPS files through our own reader (host-only code path, no GPU needed)
-    ref = "/root/reference/examples"
-    if os.path.isdir(ref):
-        import clp_b200
+    # the reference's example MPS files (kept here verbatim) through our own reader (host-only code
+    # path, no GPU needed)
+    import clp_b200
 
-        for fn in ("modified_afiro.mps", "hello.mps"):
-            s = clp_b200.ClpSimplex()
-            assert s.readMps(os.path.join(ref, fn)) == 0
-            lp = s.getProblem()
-            lp.name = fn.replace(".mps", "")
-            cases.append(lp)
+    for fn in ("modified_afiro.mps", "hello.mps"):
+        s = clp_b200.ClpSimplex()
+        assert s.readMps(os.path.join(HERE, fn)) == 0
+        lp = s.getProblem()
+        lp.name = fn.replace(".mps", "")
+        cases.append(lp)
     manifest = {}
     for lp in cases:
         src = "reference"

@@ -387,28 +387,38 @@ def test_mps_reader_rejects_unknown_names(tmp_path):
     assert clp_b200.ClpSimplex().readMps(tmp_path / "missing.mps") == -1
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples"), reason="reference tree absent")
 def test_mps_reader_on_reference_files():
+    """the reference's own example files (examples/modified_afiro.mps, examples/hello.mps), kept
+    verbatim in tests/golden/"""
     import clp_b200
 
     for fn, name in (("modified_afiro.mps", "modified_afiro"), ("hello.mps", "hello")):
         s = clp_b200.ClpSimplex()
-        assert s.readMps(os.path.join("/root/reference/examples", fn)) == 0
+        assert s.readMps(os.path.join(ROOT, "tests", "golden", fn)) == 0
         got, ref = s.getProblem(), load_golden(name)
         assert abs(got.to_scipy() - ref.to_scipy()).max() == 0
         np.testing.assert_array_equal(got.row_lower, ref.row_lower)
 
 
 def test_no_device_fails_loudly():
-    import clp_b200
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    s = clp_b200.ClpSimplex()
-    s.loadLP(load_golden("NQueens-8"))
-    with pytest.raises(clp_b200.NoDeviceError):
-        s.dual()
+    """no visible CUDA device: dual() raises instead of falling back to a CPU path.  Run in a child
+    process with the devices hidden, so that machines with a GPU check it as well."""
+    code = r"""
+import sys
+sys.path[:0] = [%r, %r]
+import clp_b200
+from conftest import load_golden
+s = clp_b200.ClpSimplex()
+s.loadLP(load_golden("NQueens-8"))
+try:
+    s.dual()
+except clp_b200.NoDeviceError:
+    print("raised NoDeviceError")
+""" % (ROOT, os.path.join(ROOT, "tests"))
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 0, out.stderr
+    assert "raised NoDeviceError" in out.stdout
 
 
 def test_two_rank_sharding_host_logic():
