@@ -50,6 +50,11 @@ SIGNATURES = {
     "Clpb_lastSolveWasHot": (ctypes.c_int, [ctypes.c_void_p]),
     "Clpb_refactorizationInterval": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "Clpb_dual": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "Clpb_primal": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "Clpb_chgObjCoefficients": (None, [ctypes.c_void_p, c_double_p]),
+    "Clpb_primalColumnPivot": (ctypes.c_int, [ctypes.c_void_p, c_double_p, c_ubyte_p, c_double_p, ctypes.c_int]),
+    "Clpb_primalRow": (ctypes.c_int, [ctypes.c_void_p, c_double_p, c_double_p, c_double_p, c_double_p, ctypes.c_int,
+                                      ctypes.c_double, ctypes.c_int, c_double_p]),
     "Clpb_status": (ctypes.c_int, [ctypes.c_void_p]),
     "Clpb_objectiveValue": (ctypes.c_double, [ctypes.c_void_p]),
     "Clpb_numberIterations": (ctypes.c_int, [ctypes.c_void_p]),

@@ -118,6 +118,7 @@ Clpb_Simplex *Clpb_presolvedModel(Clpb_Simplex *model, int *status)
   red->e.usePriceTma = model->e.usePriceTma;
   red->e.factorMode = model->e.factorMode;
   red->e.dualRowPivot = model->e.dualRowPivot;
+  red->e.primalColumnPivot = model->e.primalColumnPivot;
   red->e.rank = model->e.rank;
   red->e.worldSize = model->e.worldSize;
   red->e.ncclComm = model->e.ncclComm;
@@ -248,6 +249,8 @@ int Clpb_setParameter(Clpb_Simplex *model, const char *key, double value)
     e.hotStart = value != 0.0;
   else if (k == "dualRowPivot")
     e.dualRowPivot = (int)value;
+  else if (k == "primalColumnPivot")
+    e.primalColumnPivot = (int)value;
   else if (k == "shardPanel")
     e.shardPanelMode = (int)value;
   else if (k == "shardMinNnzPerRank")
@@ -291,6 +294,23 @@ int Clpb_refactorizationInterval(Clpb_Simplex *model, int nucleusSize) { return 
 int Clpb_dual(Clpb_Simplex *model, int)
 {
   return guarded([&] { return model->e.dual(); });
+}
+int Clpb_primal(Clpb_Simplex *model, int)
+{
+  return guarded([&] { return model->e.primal(); });
+}
+void Clpb_chgObjCoefficients(Clpb_Simplex *model, const double *obj) { model->e.chgObjCoefficients(obj); }
+int Clpb_primalColumnPivot(Clpb_Simplex *model, const double *dj, const unsigned char *status,
+                           const double *weights, int mode)
+{
+  return guarded([&] { return model->e.primalColumnPivotTest(dj, status, weights, mode); });
+}
+int Clpb_primalRow(Clpb_Simplex *model, const double *alpha, const double *xB, const double *lowerB,
+                   const double *upperB, int direction, double enteringRange, int phase, double *theta)
+{
+  return guarded([&] {
+    return model->e.primalRowTest(alpha, xB, lowerB, upperB, direction, enteringRange, phase, theta);
+  });
 }
 int Clpb_status(Clpb_Simplex *model) { return model->e.problemStatus; }
 double Clpb_objectiveValue(Clpb_Simplex *model) { return model->e.objectiveValue; }

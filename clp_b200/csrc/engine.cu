@@ -51,6 +51,9 @@ void Engine::freeAll()
   if (iterGraph)
     cudaGraphExecDestroy(iterGraph);
   iterGraph = nullptr;
+  if (primalGraph)
+    cudaGraphExecDestroy(primalGraph);
+  primalGraph = nullptr;
   if (hState)
     cudaFreeHost(hState);
   if (hRec)
@@ -486,6 +489,12 @@ int Engine::setupDevice()
   d.zeroTolerance = zeroTolerance;
   d.flagged = dalloc<unsigned char>(m);
   d.dantzig = dualRowPivot == 1 ? 1 : 0;
+  d.devex = dalloc<double>(nm);
+  d.devexRef = dalloc<unsigned char>(nm);
+  d.colFlagged = dalloc<unsigned char>(nm);
+  CUDA_OK(cudaMemset(d.colFlagged, 0, nm));
+  d.ratioPart = dalloc<double>((m + 255) / 256 + 1);
+  d.primalDantzig = 0;
   d.shardW = 1;
   d.shardPanel = 0;
   d.shardRank = 0;
@@ -1186,6 +1195,7 @@ int Engine::hotPrepare()
 int Engine::startup()
 {
   setupDevice();
+  uploadPendingCosts();
   resetStateForRun();
   largestPerturbation = 0.0;
   if (perturbation <= 100) {
@@ -1217,7 +1227,8 @@ int Engine::dual()
   if (m == 0 || n == 0)
     return trivialSolve();
   driftMeasured = false;
-  lastSolveWasHot = hotStart && deviceReady && factorsValid;
+  // a cost change leaves the basis dual infeasible: the bound-change hot start does not apply
+  lastSolveWasHot = hotStart && deviceReady && factorsValid && !costsPending;
   if ((lastSolveWasHot ? hotPrepare() : startup()) != 0) {
     problemStatus = 4;
     return problemStatus;
@@ -1836,6 +1847,306 @@ void Engine::getDeviceVector(const char *name, double *out)
     for (int i = 0; i < nm; i++)
       out[i] = st[i];
   }
+}
+
+// ---------------------------------------------------------------------------------------
+// primal simplex (ClpSimplexPrimal::primal, src/ClpSimplexPrimal.cpp; kernels in primal.cu)
+
+void Engine::chgObjCoefficients(const double *obj)
+{
+  for (int j = 0; j < n; j++)
+    hCost[j] = obj[j];
+  if (!deviceReady)
+    return; // the device copy is made from hCost at the next solve
+  wCost = hCost;
+  if (!columnScale.empty())
+    for (int j = 0; j < n; j++)
+      wCost[j] *= columnScale[j];
+  costsPending = true;
+}
+
+void Engine::uploadPendingCosts()
+{
+  if (!costsPending)
+    return;
+  CUDA_OK(cudaMemcpy(d.costTrue, wCost.data(), sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.cost, wCost.data(), sizeof(double) * nm, cudaMemcpyHostToDevice));
+  costsPending = false;
+}
+
+// Phase from the sum of infeasibilities of the basics, then that phase's costs and the duals through
+// the current factors (eta file included).  Devex is reset on request and whenever the phase changes.
+void Engine::primalCosts(bool resetDevex)
+{
+  launch_objective(d, dObj, stream);
+  double obj2[2];
+  CUDA_OK(cudaMemcpyAsync(obj2, dObj, sizeof(double) * 2, cudaMemcpyDeviceToHost, stream));
+  CUDA_OK(cudaStreamSynchronize(stream));
+  sumPrimalInfeasibilities = obj2[1];
+  const int phase = obj2[1] > 0.0 ? 1 : 2;
+  if (phase != primalPhase)
+    resetDevex = true;
+  primalPhase = phase;
+  CUDA_OK(cudaMemcpyAsync(&d.st->primalPhase, &primalPhase, sizeof(int), cudaMemcpyHostToDevice, stream));
+  launch_primal_costs(d, phase, stream);
+  launch_compute_duals(d, dPi, dZ, stream, true);
+  if (resetDevex)
+    launch_primal_devex_reset(d, stream);
+  kernelLaunches += 12;
+  CUDA_OK(cudaStreamSynchronize(stream));
+}
+
+int Engine::primalRecompute(bool resetDevex)
+{
+  launch_compute_primals(d, dXn, dRhs, stream, true);
+  kernelLaunches += 12;
+  primalCosts(resetDevex);
+  return 0;
+}
+
+// refactor -> computePrimals -> phase costs -> computeDuals -> Devex reset (no make_dual_feasible: that
+// is the dual's and moves x)
+int Engine::primalRefresh()
+{
+  if (refactor() != 0)
+    return -1;
+  currentCycle = std::min(cycleFor(d.k), d.tmax);
+  return primalRecompute(true);
+}
+
+void Engine::buildPrimalGraph()
+{
+  if (primalGraph)
+    return;
+  cudaGraph_t graph = nullptr;
+  bool ok = cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
+  if (ok) {
+    try {
+      launch_primal_iteration(d, stream);
+    } catch (const std::exception &) {
+      ok = false;
+    }
+    if (cudaStreamEndCapture(stream, &graph) != cudaSuccess || graph == nullptr)
+      ok = false;
+  }
+  if (ok) {
+    size_t numNodes = 0;
+    cudaGraphGetNodes(graph, nullptr, &numNodes);
+    primalKernelsPerIteration = (int)numNodes;
+    if (cudaGraphInstantiate(&primalGraph, graph, 0) != cudaSuccess) {
+      primalGraph = nullptr;
+      ok = false;
+    }
+  }
+  if (graph)
+    cudaGraphDestroy(graph);
+  if (!ok) {
+    cudaGetLastError(); // clear the sticky capture error
+    fprintf(stderr, "clp_b200: CUDA graph capture of the primal iteration failed, launching kernels directly\n");
+    useGraph = false;
+  }
+}
+
+// ClpSimplex::primal (src/ClpSimplex.cpp:6145) -> ClpSimplexPrimal::primal: startup, loop, finish.
+int Engine::primal()
+{
+  auto t0 = std::chrono::steady_clock::now();
+  problemStatus = -1;
+  numberIterations = 0;
+  numberRefactorizations = 0;
+  kernelLaunches = 0;
+  phase = PhaseTimes();
+  if (worldSize > 1) {
+    fprintf(stderr, "clp_b200: primal() does not run on a column-sharded model\n");
+    problemStatus = 4;
+    return problemStatus;
+  }
+  if (m == 0 || n == 0)
+    return trivialSolve();
+  driftMeasured = false;
+  lastSolveWasHot = hotStart && deviceReady && factorsValid;
+  if (lastSolveWasHot) {
+    // keep factors, eta file, x_B and status; new costs (and bounds) in force, duals recomputed
+    uploadPendingCosts();
+    boundsToWorking();
+    CUDA_OK(cudaMemcpyAsync(d.lowerTrue, wLower.data(), sizeof(double) * nm, cudaMemcpyHostToDevice, stream));
+    CUDA_OK(cudaMemcpyAsync(d.upperTrue, wUpper.data(), sizeof(double) * nm, cudaMemcpyHostToDevice, stream));
+    CUDA_OK(cudaMemsetAsync(&d.st->stop, 0, sizeof(int), stream));
+    CUDA_OK(cudaMemsetAsync(&d.st->pchuzcKey, 0, sizeof(unsigned long long), stream));
+    launch_primal_bounds(d, stream);
+  } else {
+    setupDevice();
+    uploadPendingCosts();
+    resetStateForRun();
+  }
+  if (primalGraph) { // DeviceModel is captured by value
+    cudaGraphExecDestroy(primalGraph);
+    primalGraph = nullptr;
+  }
+  d.primalDantzig = primalColumnPivot == 1 ? 1 : 0;
+  setAcceptablePivot(acceptablePivot);
+  primalPhase = 0; // decided from the first sum of infeasibilities
+  if ((lastSolveWasHot ? primalRecompute(true) : primalRefresh()) != 0) {
+    problemStatus = 4;
+    return problemStatus;
+  }
+  int consecutiveTrouble = 0, lastBadColumn = -1, confirmations = 0;
+  while (problemStatus < 0) {
+    if (numberIterations >= maximumIterations) {
+      problemStatus = 3;
+      break;
+    }
+    if (std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count() > maximumSeconds) {
+      problemStatus = 3;
+      break;
+    }
+    fetchState();
+    const int room = std::min(currentCycle, d.tmax) - hState->numEtas;
+    if (room <= 0) {
+      if (primalRefresh() != 0)
+        problemStatus = 4;
+      continue;
+    }
+    int count = std::min(std::min(batch, room), maximumIterations - numberIterations);
+    count = std::min(count, d.recCap);
+    const int before = hState->iterations;
+    launch_primal_chuzc(d, stream);
+    kernelLaunches += 2;
+    if (useGraph)
+      buildPrimalGraph(); // may clear useGraph
+    if (useGraph) {
+      for (int b = 0; b < count; b++)
+        CUDA_OK(cudaGraphLaunch(primalGraph, stream));
+      kernelLaunches += (long)count * primalKernelsPerIteration;
+    } else {
+      for (int b = 0; b < count; b++)
+        launch_primal_iteration(d, stream);
+    }
+    fetchState();
+    const int done = hState->iterations - before;
+    numberIterations += done;
+    if (logLevel > 1)
+      fprintf(stderr, "clp_b200: primal it %d etas %d phase %d stop %d\n", numberIterations, hState->numEtas,
+              primalPhase, hState->stop);
+    const int stop = hState->stop;
+    if (stop == STOP_NONE) {
+      consecutiveTrouble = 0;
+      continue;
+    }
+    CUDA_OK(cudaMemsetAsync(&d.st->stop, 0, sizeof(int), stream));
+    const bool fresh = hState->numEtas == 0;
+    switch (stop) {
+    case STOP_ETAS_FULL:
+      if (primalRefresh() != 0)
+        problemStatus = 4;
+      break;
+    case STOP_PHASE_COSTS: // phase 1: the infeasibility set changed (ClpSimplexPrimal::pivotColumn updates)
+      primalCosts(false);
+      break;
+    case STOP_INACCURATE: {
+      if (++consecutiveTrouble > 50) {
+        problemStatus = 4;
+        break;
+      }
+      const int q = hState->seqIn;
+      if (!fresh && primalRefresh() != 0) {
+        problemStatus = 4;
+        break;
+      }
+      if (fresh || q == lastBadColumn) {
+        // the same column fails on fresh factors: leave it out until the next refactorization
+        const unsigned char one = 1;
+        CUDA_OK(cudaMemcpy(d.colFlagged + q, &one, 1, cudaMemcpyHostToDevice));
+      }
+      lastBadColumn = q;
+      break;
+    }
+    case STOP_NO_COLUMN:
+    case STOP_UNBOUNDED:
+      // believed only on fresh factors with recomputed primals and duals, and without flagged columns
+      if (!fresh || (lastBadColumn >= 0 && confirmations < 3)) {
+        confirmations++;
+        lastBadColumn = -1;
+        if (primalRefresh() != 0)
+          problemStatus = 4;
+        break;
+      }
+      if (stop == STOP_NO_COLUMN)
+        problemStatus = primalPhase == 2 ? 0 : 1;
+      else
+        problemStatus = primalPhase == 2 ? 2 : 4;
+      break;
+    default:
+      problemStatus = 4;
+      break;
+    }
+  }
+  // leave the device state as a dual hot start expects it: true costs, unit dual weights
+  CUDA_OK(cudaMemcpyAsync(d.cost, d.costTrue, sizeof(double) * nm, cudaMemcpyDeviceToDevice, stream));
+  if (problemStatus != 0) // optimal: the duals already belong to the true costs
+    launch_compute_duals(d, dPi, dZ, stream, true);
+  std::vector<double> w(m, 1.0);
+  CUDA_OK(cudaMemcpyAsync(d.weights, w.data(), sizeof(double) * m, cudaMemcpyHostToDevice, stream));
+  downloadSolution();
+  secondsInLoop = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  return problemStatus;
+}
+
+int Engine::primalColumnPivotTest(const double *dj, const unsigned char *stat, const double *weights, int mode)
+{
+  setupDevice();
+  resetStateForRun();
+  CUDA_OK(cudaMemcpy(d.dj, dj, sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.status, stat, nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.devex, weights, sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemset(d.colFlagged, 0, nm));
+  DeviceModel dm = d;
+  dm.primalDantzig = mode == 1 ? 1 : 0;
+  launch_primal_chuzc(dm, stream);
+  fetchState();
+  return hState->stop != 0 ? -1 : hState->seqIn;
+}
+
+// The ratio test on explicit vectors: position p holds a basic slack (sequence n+p) with value xB[p] and
+// bounds lowerB[p] / upperB[p]; the entering variable is column 0 with range enteringRange.
+int Engine::primalRowTest(const double *alpha, const double *xB, const double *lowerB, const double *upperB,
+                          int direction, double enteringRange, int phase, double *theta)
+{
+  setupDevice();
+  resetStateForRun();
+  std::vector<double> lo(wLower), up(wUpper), x(nm, 0.0);
+  std::vector<int> pv(m);
+  std::vector<unsigned char> ref(nm, 0);
+  for (int p = 0; p < m; p++) {
+    pv[p] = n + p;
+    x[n + p] = xB[p];
+    lo[n + p] = lowerB[p] < -1.0e29 ? -kInf : lowerB[p];
+    up[n + p] = upperB[p] > 1.0e29 ? kInf : upperB[p];
+  }
+  lo[0] = 0.0;
+  up[0] = enteringRange > 1.0e29 ? kInf : enteringRange;
+  CUDA_OK(cudaMemcpy(d.lower, lo.data(), sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.upper, up.data(), sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.sol, x.data(), sizeof(double) * nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.pivotVariable, pv.data(), sizeof(int) * m, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.devexRef, ref.data(), nm, cudaMemcpyHostToDevice));
+  CUDA_OK(cudaMemcpy(d.rhs3, alpha, sizeof(double) * m, cudaMemcpyHostToDevice));
+  IterState st;
+  memset(&st, 0, sizeof(st));
+  st.seqIn = 0;
+  st.primalDir = direction < 0 ? -1 : 1;
+  st.primalPhase = phase == 1 ? 1 : 2;
+  st.acceptablePivot = acceptablePivot;
+  st.ratioBits = 0x7FF0000000000000ull;
+  CUDA_OK(cudaMemcpy(d.st, &st, sizeof(st), cudaMemcpyHostToDevice));
+  launch_primal_ratio(d, stream);
+  fetchState();
+  if (hState->stop == STOP_UNBOUNDED) {
+    *theta = kInf;
+    return -1;
+  }
+  *theta = std::fabs(hState->thetaPrimal);
+  return hState->primalFlip ? -2 : hState->pivotRow;
 }
 
 } // namespace clpb

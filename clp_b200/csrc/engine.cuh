@@ -41,8 +41,12 @@ constexpr int kPriceTileAlloc = kPriceTile + 8;
 constexpr int kPriceTileCols = 8;         // columns per tile (one warp each)
 
 // stop reasons written by the device into IterState.stop
+// (primal simplex: STOP_NO_COLUMN = no entering column, STOP_UNBOUNDED = no blocking row and an
+// entering variable without a finite range, STOP_PHASE_COSTS = a basic variable changed its
+// infeasibility state in phase 1, so the phase-1 costs and the duals must be recomputed)
 enum : int { STOP_NONE = 0, STOP_NO_ROW = 1, STOP_NO_COLUMN = 2, STOP_INACCURATE = 3,
-             STOP_ETAS_FULL = 4, STOP_TINY_PIVOT = 5, STOP_FLIPS_OVERFLOW = 6 };
+             STOP_ETAS_FULL = 4, STOP_TINY_PIVOT = 5, STOP_FLIPS_OVERFLOW = 6, STOP_UNBOUNDED = 7,
+             STOP_PHASE_COSTS = 8 };
 
 // Per-iteration scalars, device resident (one instance).  Every kernel of the iteration reads
 // what it needs from here, so the launch sequence is independent of the pivot choices and
@@ -77,6 +81,16 @@ struct IterState {
   // iteration graph holds DeviceModel by value
   double acceptablePivot;
   int numFlagged;        // rows currently excluded from CHUZR (ClpSimplex::setFlagged, ClpSimplexDual.cpp:2058-2066)
+  // primal simplex (primal.cu)
+  int primalDir;         // +1 the entering variable increases, -1 it decreases
+  int primalFlip;        // 1: this iteration moves the entering variable to its other bound (no basis change)
+  int primalPhase;       // 1 sum of infeasibilities, 2 true costs
+  int infeasChanged;     // phase 1: a basic variable changed its infeasibility state in this iteration
+  double primalDj;       // d_q of the entering variable
+  double devexQ;         // reference weight of the entering column, exact from its FTRAN
+  unsigned long long pchuzcKey; // packed (score, sequence) argmax of the primal CHUZC
+  unsigned long long ratioBits; // relaxed minimum step of the ratio test (double bits, positive)
+  unsigned long long ratioKey;  // packed (|alpha|, position) argmax of the second ratio-test pass
 };
 
 struct IterRecord { // what the host reads back per iteration
@@ -181,6 +195,12 @@ struct DeviceModel {
   double *gatherB; // [W][shardPerK]     BTRAN GEMV results
   double *gatherP; // [W][3][shardPerM]  eta-panel results
   unsigned char *flagged; // [m] by position: 1 = row is flagged (skipped by CHUZR until the next refactorization)
+  // primal simplex (primal.cu)
+  double *devex;             // [n+m] Devex weights by sequence (ClpPrimalColumnSteepest::weights_)
+  unsigned char *devexRef;   // [n+m] 1 = in the Devex reference framework (nonbasic at the last reset)
+  unsigned char *colFlagged; // [n+m] 1 = excluded from the primal CHUZC until the next refactorization
+  double *ratioPart;         // [m/256+1] per-CTA partial sums of the entering column's reference weight
+  int primalDantzig;         // primalColumnPivot: 0 Devex, 1 Dantzig
 };
 
 // Optional per-kernel CUDA-event brackets (timing mode only): price kernel, FTRAN GEMV, BTRAN GEMV.
@@ -234,6 +254,13 @@ void launch_gather_nucleus_matrix(const DeviceModel &d, double *N, int ld, cudaS
 void launch_count_fake(const DeviceModel &d, int *counter, cudaStream_t s);
 void launch_unpack_column(const DeviceModel &d, int seq, double *out, cudaStream_t s);
 void launch_eta_append_test(const DeviceModel &d, int pivotRow, int seqIn, cudaStream_t s);
+// primal.cu
+void launch_primal_chuzc(const DeviceModel &d, cudaStream_t s);  // stand-alone CHUZC (start of a batch)
+void launch_primal_ratio(const DeviceModel &d, cudaStream_t s);  // Harris two-pass ratio test over x_B
+void launch_primal_iteration(const DeviceModel &d, cudaStream_t s); // one whole primal iteration
+void launch_primal_costs(const DeviceModel &d, int phase, cudaStream_t s); // phase-1 or true costs into d.cost
+void launch_primal_devex_reset(const DeviceModel &d, cudaStream_t s);
+void launch_primal_bounds(const DeviceModel &d, cudaStream_t s); // true bounds in force, nonbasics at them
 // factor.cu
 int dense_invert(double *A, double *X, int k, int ld, int *dIpiv, int *dPerm, int *dInfo,
                  int *hostIpiv, int *hostPerm, double singularTol, cudaStream_t s, int shardW = 1,

@@ -97,6 +97,18 @@ public:
   void chgBounds(const double *columnLower, const double *columnUpper, const double *rowLower,
                  const double *rowUpper); // NULL = unchanged
   bool lastSolveWasHot = false;
+  // ---- solve (ClpSimplex::primal, src/ClpSimplex.cpp:6145; primal.cu) ----
+  // Phase 1 minimises the sum of infeasibilities, phase 2 the true costs; "perturbation" is ignored.
+  // With hotStart set, a primal() that follows a solve of the same model keeps the device-resident
+  // factors, eta file, x_B and status, recomputes the duals for the (changed) costs and iterates.
+  int primal();
+  int primalColumnPivot = 0; // ClpSimplex::setPrimalColumnPivotAlgorithm: 0 exact Devex, 1 Dantzig
+  // Clp_chgObjCoefficients (src/Clp_C_Interface.h:158): replaces the loaded objective (n entries)
+  void chgObjCoefficients(const double *obj);
+  // plug-in entries on explicit host vectors (ClpPrimalColumnPivot::pivotColumn, ClpSimplexPrimal::primalRow)
+  int primalColumnPivotTest(const double *dj, const unsigned char *stat, const double *weights, int mode);
+  int primalRowTest(const double *alpha, const double *xB, const double *lowerB, const double *upperB,
+                    int direction, double enteringRange, int phase, double *theta);
   int cycleFor(int k) const; // refactorization interval the default policy uses at nucleus size k (host only)
   int problemStatus = -1;
   int numberIterations = 0, numberRefactorizations = 0;
@@ -167,6 +179,15 @@ private:
   bool factorsValid = false; // a factorization of the current device basis exists
   void boundsToWorking();    // hLower/hUpper -> wLower/wUpper with the scale factors in force
   int hotPrepare();
+  bool costsPending = false; // chgObjCoefficients after the device copy was made: costTrue is stale
+  void uploadPendingCosts();
+  int primalPhase = 1;
+  int primalRefresh();             // refactor + primalRecompute
+  int primalRecompute(bool resetDevex); // computePrimals, phase + costs, computeDuals (current factors)
+  void primalCosts(bool resetDevex);    // phase from the sum of infeasibilities, its costs, computeDuals
+  cudaGraphExec_t primalGraph = nullptr; // one captured primal iteration
+  int primalKernelsPerIteration = 0;
+  void buildPrimalGraph();
   long long readySignature = -1;
   int trivialSolve(); // m == 0 or n == 0 (a presolved model can be empty): host only
   bool haveUserStatus = false;

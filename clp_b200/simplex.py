@@ -113,6 +113,17 @@ class ClpSimplex:
         self.postsolve(red)  # also hands a non-optimal status back to this model
         return rc
 
+    def initialPrimalSolve(self, presolve=True):
+        """ClpSimplex::initialSolve with the primal algorithm: presolve -> primal -> postsolve."""
+        if not presolve:
+            return self.primal()
+        st, red = self.presolvedModel()
+        if red is None:
+            return st
+        rc = red.primal()
+        self.postsolve(red)
+        return rc
+
     def writeMps(self, fileName, formatType=1, numberAcross=1, objSense=0.0):
         return self._L.Clpb_writeMps(self._h, str(fileName).encode(), int(formatType), int(numberAcross), float(objSense))
 
@@ -204,6 +215,27 @@ class ClpSimplex:
         if rc == -99:
             raise RuntimeError("clp_b200: CUDA failure inside dual()")
         return rc
+
+    # ---- ClpSimplex::primal ----
+    def primal(self, ifValuesPass=0):
+        """ClpSimplex::primal (phase 1 sum of infeasibilities, Devex or Dantzig pricing)."""
+        rc = self._L.Clpb_primal(self._h, int(ifValuesPass))
+        if rc == _capi.NO_DEVICE:
+            raise NoDeviceError("clp_b200 needs a CUDA device (no CPU fallback)")
+        if rc == -99:
+            raise RuntimeError("clp_b200: CUDA failure inside primal()")
+        return rc
+
+    def chgObjCoefficients(self, obj):
+        """Clp_chgObjCoefficients: replace the loaded objective (n entries)."""
+        o = np.ascontiguousarray(obj, dtype=np.float64)
+        if o.shape != (self.numberColumns(),):
+            raise ValueError("chgObjCoefficients needs one cost per column")
+        self._L.Clpb_chgObjCoefficients(self._h, _dp(o))
+
+    def setPrimalColumnPivotAlgorithm(self, mode):
+        """0 exact Devex (default), 1 Dantzig."""
+        self._set("primalColumnPivot", mode)
 
     def status(self): return self._L.Clpb_status(self._h)
     def isProvenOptimal(self): return self.status() == 0
@@ -378,6 +410,21 @@ class ClpSimplex:
         self._chk(self._L.Clpb_transposeTimesPacked(self._h, float(scalar), len(ip), _ip(ip), _dp(ep),
                                                     ctypes.byref(nz), _ip(iz), _dp(ez)))
         return iz[:nz.value].copy(), ez[:nz.value].copy()
+
+    def primalColumnPivot(self, dj, status, weights, mode=0):
+        """ClpPrimalColumnPivot::pivotColumn on explicit dj / status / weights (n+m each) -> sequence or -1"""
+        d = np.ascontiguousarray(dj, dtype=np.float64)
+        s = np.ascontiguousarray(status, dtype=np.uint8)
+        w = np.ascontiguousarray(weights, dtype=np.float64)
+        return self._chk(self._L.Clpb_primalColumnPivot(self._h, _dp(d), _up(s), _dp(w), int(mode)))
+
+    def primalRow(self, alpha, xB, lowerB, upperB, direction, enteringRange, phase=2):
+        """ClpSimplexPrimal::primalRow on explicit vectors (m each) -> (row, -1 no block or -2 flip; theta)"""
+        a, x, lo, up = (np.ascontiguousarray(v, dtype=np.float64) for v in (alpha, xB, lowerB, upperB))
+        theta = ctypes.c_double(0.0)
+        r = self._chk(self._L.Clpb_primalRow(self._h, _dp(a), _dp(x), _dp(lo), _dp(up), int(direction),
+                                             float(enteringRange), int(phase), ctypes.byref(theta)))
+        return r, theta.value
 
     def startup(self): return self._chk(self._L.Clpb_startup(self._h))
     def iterate(self, count): return self._chk(self._L.Clpb_iterate(self._h, int(count)))

@@ -60,7 +60,7 @@ void Clpb_getProblem(Clpb_Simplex *model, int *start, int *index, double *value,
 /* Clp_setPrimalTolerance :179, Clp_setDualTolerance :182, Clp_setDualBound :382,
    Clp_setMaximumIterations :199, Clp_setMaximumSeconds :202, Clp_setLogLevel :314,
    ClpFactorization::maximumPivots (src/ClpFactorization.hpp:149).  Keys: "primalTolerance",
-   "dualTolerance", "dualBound", "maximumIterations", "maximumSeconds", "logLevel",
+   "dualTolerance", "dualBound", "maximumIterations", "maximumSeconds", "logLevel", "primalColumnPivot",
    "factorizationFrequency", "scaling", "perturbation" (Clp_setPerturbation :395: 50 on,
    100 automatic, 102 off = default here; ClpSimplexDual::perturb src/ClpSimplexDual.cpp:6533), "batch" (iterations enqueued per host sync), "timing" (0/1: per-phase
    CUDA events, no graph replay), "useGraph" (0/1), "warmupIterations", "objectiveOffset". */
@@ -107,6 +107,19 @@ int Clpb_refactorizationInterval(Clpb_Simplex *model, int nucleusSize);
    0 optimal, 1 primal infeasible, 2 dual infeasible, 3 stopped on iterations/time,
    4 stopped due to errors. */
 int Clpb_dual(Clpb_Simplex *model, int ifValuesPass);
+/* Clp_primal :348 (ClpSimplex::primal src/ClpSimplex.cpp:6145).  Same return codes as Clpb_dual.
+   Phase 1 minimises the sum of infeasibilities, phase 2 the loaded costs; pricing by the key
+   "primalColumnPivot" (ClpSimplex::setPrimalColumnPivotAlgorithm): 0 exact Devex
+   (ClpPrimalColumnSteepest mode 0, the default), 1 Dantzig (ClpPrimalColumnDantzig).  The values pass
+   is not built: ifValuesPass != 0 is treated as 0.  "perturbation" is ignored.  A model with
+   sharding initialised (Clpb_initSharding, worldSize > 1) is refused with 4.  With "hotStart" = 1 a
+   Clpb_primal that follows a solve of the same model keeps the factors, eta file, x_B and status on
+   the device, recomputes the duals for the costs now loaded and iterates (Clpb_lastSolveWasHot says
+   so): the re-solve after Clpb_chgObjCoefficients. */
+int Clpb_primal(Clpb_Simplex *model, int ifValuesPass);
+/* Clp_chgObjCoefficients :158: obj[n] replaces the loaded objective (Clpb_getProblem returns it; the
+   device copy is updated at the next solve).  A hot Clpb_dual is not taken after a cost change. */
+void Clpb_chgObjCoefficients(Clpb_Simplex *model, const double *obj);
 int Clpb_status(Clpb_Simplex *model);
 /* Clp_objectiveValue :256, Clp_numberIterations :195 */
 double Clpb_objectiveValue(Clpb_Simplex *model);
@@ -180,6 +193,21 @@ int Clpb_dualColumn(Clpb_Simplex *model, const double *alphaRow, const double *d
 int Clpb_dualColumnRowPass(Clpb_Simplex *model, const double *alphaRow, const double *dj,
                            const unsigned char *status, int direction, double infeasibility,
                            double *theta);
+/* ClpPrimalColumnPivot::pivotColumn (src/ClpPrimalColumnPivot.hpp) on explicit vectors dj[n+m],
+   status[n+m], weights[n+m]; mode 0 Devex (score dj^2/weight), 1 Dantzig (dj^2).  Candidates: at lower
+   with dj < -dualTolerance, at upper with dj > dualTolerance, free / superbasic with |dj| > dualTolerance.
+   Returns the entering sequence or -1.  Scores that agree in their upper 44 bits: the smaller sequence. */
+int Clpb_primalColumnPivot(Clpb_Simplex *model, const double *dj, const unsigned char *status,
+                           const double *weights, int mode);
+/* ClpSimplexPrimal::primalRow (src/ClpSimplexPrimal.cpp:1877), Harris two-pass ratio test on explicit
+   vectors: alpha[m] = B^-1 a_q, basic values xB[m] with bounds lowerB[m] / upperB[m]; the entering
+   variable moves up (direction +1) or down (-1) and has range enteringRange (>= 1e30: none).  phase 1:
+   infeasible basics block only at their far bound.  Returns the pivot row, -1 no block (unbounded ray), or
+   -2 the entering variable reaches its other bound first; *theta = the step (>= 0).  Pivots below
+   "acceptablePivot" are ignored; among the rows within the relaxed step the largest |alpha| wins
+   (ties: the smaller row). */
+int Clpb_primalRow(Clpb_Simplex *model, const double *alpha, const double *xB, const double *lowerB,
+                   const double *upperB, int direction, double enteringRange, int phase, double *theta);
 /* The dense kernel of the refactorization on its own (CoinAbcDgetrf + inverse,
    src/AbcSimplexParallel.cpp:2491): a[k*k] column-major in, x = a^-1 column-major out.
    Returns 0, or 1 + the index of the first column without an acceptable pivot. */
